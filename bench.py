@@ -11,6 +11,7 @@ with HOST buffers: pinned actions -> device, control law, step, qpos/qvel -> pin
     python -m torch.distributed.run --nnodes=1 --nproc-per-node 8 --master-addr 127.0.0.1 \
         --master-port 29500 bench.py --gpus 8 --steps 20 --warmup 3
     python bench.py --impl reference        # the CPU port of the reference path on the host cores
+    python bench.py --dump-outputs bench_outputs     # also write what the last timed step computed, bench_outputs/<name>.npy
 """
 import argparse
 import json
@@ -656,6 +657,28 @@ class RearrangeTcpWorkload(RearrangeWorkload):
         return self.torch.rand(self.sim.nenv, 6, device=self.dev, generator=self.gen) * 2 - 1
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(arrays, out_dir, limit=DUMP_LIMIT_BYTES, seed=0):
+    """Write each [nenv, ...] array as out_dir/<name>.npy: float32 arrays as they are, integer ones as float64 (exact).
+    When they would take more than `limit` bytes in all, the same fixed, seeded sample of environments is taken from every
+    array and its indices are written as env_index.npy."""
+    import numpy as np
+
+    arrays = {k: v.cpu().numpy() for k, v in arrays.items()}
+    arrays = {k: v.astype(np.float32 if v.dtype == np.float32 else np.float64) for k, v in arrays.items()}
+    nenv = next(iter(arrays.values())).shape[0]
+    per_env = sum(v.nbytes // nenv for v in arrays.values())
+    if per_env * nenv > limit:
+        rows = np.sort(np.random.RandomState(seed).choice(nenv, max(1, (limit - 8 * nenv) // per_env), replace=False))
+        arrays = {k: v[rows] for k, v in arrays.items()}
+        arrays["env_index"] = rows.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
+
+
 def run_gpu_arm(args):
     import numpy as np
     import torch
@@ -690,8 +713,8 @@ def run_gpu_arm(args):
     nsub = cfg.get("nsub", NSUB)
     rearrange = cfg.get("workload") in ("rearrange", "rearrange_tcp")
     tcp = cfg.get("workload") == "rearrange_tcp"
-    sim = engine.BatchedSim(model, N, nsub, outputs=("site_xpos", "act_force", "ncon", "warn") + (("body_xpos", "body_xquat") if rearrange else ()),
-                            contact_capacity=caps[0], row_capacity=caps[1], dofs_per_contact=caps[2])
+    outputs = ("site_xpos", "act_force", "ncon", "warn") + (("body_xpos", "body_xquat") if rearrange else ())
+    sim = engine.BatchedSim(model, N, nsub, outputs=outputs, contact_capacity=caps[0], row_capacity=caps[1], dofs_per_contact=caps[2])
     m = model.host
     nu, nq, nv = m["nu"], m["nq"], m["nv"]
     gen = torch.Generator(device=dev)
@@ -742,6 +765,7 @@ def run_gpu_arm(args):
     ncon_sum = torch.zeros((), dtype=torch.float64, device=dev)
     warn = torch.zeros((), dtype=torch.int32, device=dev)
     ncon_max = torch.zeros((), dtype=torch.int32, device=dev)
+    last = None
     for k in range(args.steps):
         nxt = wl.sample_action()
         flush.zero_()                                   # evict L2 between timed iterations (outside the event pair)
@@ -750,6 +774,10 @@ def run_gpu_arm(args):
         ev[k][0].record()
         wl.step_timed()                                 # one launch (two for the dual-simulation rearrange loop, hand-off included)
         ev[k][1].record()
+        if args.dump_outputs and k == args.steps - 1:   # what the last timed step handed its caller, before the auto-reset
+            last = {n: getattr(sim, n).clone() for n in ("qpos", "qvel", "ctrl") + outputs}
+            if solver is not None:
+                last.update({"solver_" + n: getattr(solver, n).clone() for n in ("qpos", "qvel", "ctrl")})
         ncon_sum += sim.ncon.double().mean()
         ncon_max = torch.maximum(ncon_max, sim.ncon.max())
         warn |= sim.warn.max() if solver is None else torch.maximum(sim.warn.max(), solver.warn.max())
@@ -848,6 +876,8 @@ def run_gpu_arm(args):
             except Exception as e:  # the baseline is reported, never required for the GPU number
                 line["cpu_baseline"] = {"value": None, "unit": "env-steps/s", "cores": 0, "kind": "port", "sample": f"failed: {e}"}
         print(json.dumps(line), flush=True)
+        if last is not None:
+            dump_outputs(last, args.dump_outputs)
     if dist is not None:
         dist.destroy_process_group()
 
@@ -868,8 +898,15 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--randomize", action="store_true", help="dactyl configs: per-environment model parameters drawn with the reference wrappers' distributions "
                                                              "(locked.py:263-277 / full_perpendicular.py:425-440), per-step timestep and wind -- SURVEY 8(d) cfg 3's randomize=True")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step of the device-resident region computed (rank 0's "
+                                                           "environments: qpos, qvel, ctrl and the engine's outputs) as DIR/<name>.npy; "
+                                                           "the inputs are seeded, so two builds can be compared output for output")
     ap.add_argument("--config", default="locked", choices=sorted(CONFIGS), help="locked = BASELINE.json's headline config; full_perpendicular = configs[2]; rearrange_blocks = configs[3]; rearrange_ycb = configs[4]")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs: the GPU path only")
     if args.impl == "reference":
         run_reference_arm(args)
     else:

@@ -1,78 +1,39 @@
-"""Batched host facade (robogym_b200/batched_env.py) against the reference's OWN per-env code, driven
-through the mujoco_py shim (oracle engine, CPU).  Build-container only: needs /root/reference."""
+"""Batched host facade (robogym_b200/batched_env.py) against the reference's OWN per-env code: robogym's locked
+environment on the mujoco_py shim (oracle engine, CPU) recorded its controls, observations, contacts and occlusion
+flags, and the model fields its randomisation wrappers changed (tests/golden/ref_facade.npz, tools/make_reference_golden.py);
+the facade must compute the same from the recorded simulator state."""
 import os
-import sys
 
 import numpy as np
-import pytest
 
-REF = os.environ.get("ROBOGYM_REFERENCE", "/root/reference")
-pytestmark = [pytest.mark.needs_reference, pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "robogym")), reason="needs /root/reference")]
+HERE = os.path.dirname(os.path.abspath(__file__))
 
 
-@pytest.fixture(scope="module")
-def ref_env():
-    here = os.path.dirname(os.path.abspath(__file__))
-    for p in (os.path.join(here, "stubs"), REF):
-        if p not in sys.path:
-            sys.path.insert(0, p)
-    import robogym_b200.mujoco_py_shim as shim
-
-    shim.install()
-    from oracle_engine import OracleEngine
-
-    shim.set_engine_factory(OracleEngine)
-    from robogym.envs.dactyl.locked import make_env
-
-    env = make_env(starting_seed=3)
-    env.reset()
-    yield env
-    shim.set_engine_factory(None)
-
-
-def test_facade_matches_reference_host_code(ref_env):
+def test_facade_matches_reference_host_code(locked_blob, locked_names):
     import torch
 
-    from robogym.utils.sensor_utils import check_occlusion
+    from robogym_b200 import modelblob
     from robogym_b200.batched_env import ShadowHandCubeFacade
 
-    env = ref_env.unwrapped
-    sim = env.mujoco_simulation.mj_sim
-    cm = sim.model._cm
-    fac = ShadowHandCubeFacade(cm.m, cm.names, "cpu", dtype=torch.float64)
-    robot = env.mujoco_simulation.shadow_hand
-    rng = np.random.RandomState(0)
-    occ_names = [n for n in cm.names["geom"] if n and n.endswith("occlusion")]
-    seen_contact = False
-    for k in range(12):
-        action = rng.uniform(-1, 1, 20)
+    g = np.load(os.path.join(HERE, "golden", "ref_facade.npz"))
+    m = modelblob.unpack(locked_blob)
+    m.update({k[len("model_"):]: g[k] for k in g.files if k.startswith("model_")})    # the recorded environment's randomised model
+    fac = ShadowHandCubeFacade(m, locked_names, "cpu", dtype=torch.float64)
+    t = lambda k, i: torch.tensor(g[k][i][None])
+    for k in range(len(g["action"])):
         # a6: relative and absolute denormalisation
-        want_rel = robot.denormalize_position_control(action, relative_action=True)
-        want_abs = robot.denormalize_position_control(action, relative_action=False)
-        q = torch.tensor(sim.data.qpos[None].copy())
-        got_rel = fac.denormalize_position_control(torch.tensor(action[None]), q, relative_action=True)[0].numpy()
-        got_abs = fac.denormalize_position_control(torch.tensor(action[None]), None, relative_action=False)[0].numpy()
-        assert np.abs(got_rel - want_rel).max() < 1e-12 and np.abs(got_abs - want_abs).max() < 1e-12
-        robot.set_position_control(want_rel)
-        env.mujoco_simulation.step()
+        got_rel = fac.denormalize_position_control(t("action", k), t("qpos_before", k), relative_action=True)[0].numpy()
+        got_abs = fac.denormalize_position_control(t("action", k), None, relative_action=False)[0].numpy()
+        assert np.abs(got_rel - g["ctrl_rel"][k]).max() < 1e-12 and np.abs(got_abs - g["ctrl_abs"][k]).max() < 1e-12
         # a7: observations
-        obs = env.observe()
-        sx = torch.tensor(sim.data.site_xpos[None].copy())
-        q, v = torch.tensor(sim.data.qpos[None].copy()), torch.tensor(sim.data.qvel[None].copy())
-        mine = fac.observe(q, v, sx, torch.tensor(sim.data.actuator_force[None].copy()))
+        sx = t("site_xpos", k)
+        mine = fac.observe(t("qpos", k), t("qvel", k), sx, t("actuator_force", k))
         for key in ("cube_pos", "cube_quat", "hand_angle", "fingertip_pos"):
-            assert np.abs(mine[key][0].numpy().ravel() - np.asarray(obs[key]).ravel()).max() < 1e-9, key
-        hand_obs = robot.observe()
-        assert np.abs(mine["actuator_force"][0].numpy() - hand_obs.actuator_effort()).max() < 1e-9
+            assert np.abs(mine[key][0].numpy().ravel() - g[key][k]).max() < 1e-9, key
+        assert np.abs(mine["actuator_force"][0].numpy() - g["effort"][k]).max() < 1e-9
         # a8
-        assert bool(fac.on_palm(sx)[0]) == bool(env.mujoco_simulation.is_cube_on_palm())
+        assert bool(fac.on_palm(sx)[0]) == bool(g["on_palm"][k])
         # a9
-        con = np.zeros((1, 64, 4))
-        for i in range(sim.data.ncon):
-            c = sim.data.contact[i]
-            con[0, i] = (c.geom1, c.geom2, c.dist, c.dim)
-        got = fac.fingers_occluded(torch.tensor(con), torch.tensor([sim.data.ncon]))[0].numpy()
-        want = np.array(check_occlusion(sim, dist_cutoff=-1e-4))
-        assert np.array_equal(got.astype(int), want.astype(int))
-        seen_contact |= sim.data.ncon > 0
-    assert seen_contact
+        got = fac.fingers_occluded(t("contact", k), torch.tensor([int(g["ncon"][k])]))[0].numpy()
+        assert np.array_equal(got.astype(int), g["occluded"][k])
+    assert (g["ncon"] > 0).any()

@@ -100,3 +100,24 @@ def test_reference_arm_prints_the_contract_line():
     assert line["cpu_baseline"]["kind"] == "port" and line["cpu_baseline"]["cores"] >= 1
     assert line["e2e"]["h2d_bytes_per_step"] == 0 and line["e2e"]["d2h_bytes_per_step"] == 0 and line["gpu_launches"] == 0
     assert "workload" in line["config"]
+
+
+def test_dump_outputs_writes_float_arrays_and_samples_environments(tmp_path):
+    """bench.py --dump-outputs: float32 outputs stay float32, integer ones become exact float64; above the size limit the same
+    seeded sample of environments is taken from every array and its indices are written beside them."""
+    import torch
+
+    import bench
+
+    n = 1000
+    arrays = dict(qpos=torch.arange(n * 3, dtype=torch.float32).reshape(n, 3), ncon=torch.arange(n, dtype=torch.int32))
+    bench.dump_outputs(arrays, str(tmp_path / "all"))
+    q, c = np.load(tmp_path / "all" / "qpos.npy"), np.load(tmp_path / "all" / "ncon.npy")
+    assert q.dtype == np.float32 and c.dtype == np.float64 and np.array_equal(q, arrays["qpos"].numpy()) and np.array_equal(c, np.arange(n))
+    assert not (tmp_path / "all" / "env_index.npy").exists()
+    for d in ("a", "b"):
+        bench.dump_outputs(arrays, str(tmp_path / d), limit=4000)
+    idx = np.load(tmp_path / "a" / "env_index.npy")
+    assert np.array_equal(idx, np.load(tmp_path / "b" / "env_index.npy")) and 0 < len(idx) < n
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in os.listdir(tmp_path / "a")) < 4000 + 3 * 128     # + .npy headers
+    assert np.array_equal(np.load(tmp_path / "a" / "ncon.npy"), idx) and np.array_equal(np.load(tmp_path / "a" / "qpos.npy")[:, 0], 3 * idx)

@@ -1,6 +1,7 @@
 """Batched dactyl/locked environment (robogym_b200/locked_env.py): goal generation, goal reward, multi-goal
-bookkeeping, drop handling and reset -- against the reference's own LockedEnv driven through the mujoco_py shim
-(build container, CPU), by itself on the CPU oracle simulator, and on the CUDA engine (gpu)."""
+bookkeeping, drop handling and reset -- against the answers of the reference's own LockedEnv driven through the mujoco_py
+shim (recorded in tests/golden/ref_locked_*.npz by tools/make_reference_golden.py), by itself on the CPU oracle simulator,
+and on the CUDA engine (gpu)."""
 import math
 import os
 import sys
@@ -11,8 +12,6 @@ import pytest
 from robogym_b200 import modelblob
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-REF = os.environ.get("ROBOGYM_REFERENCE", "/root/reference")
-needs_reference = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "robogym")), reason="needs /root/reference")
 sys.path.insert(0, os.path.join(HERE, "stubs"))
 
 
@@ -27,135 +26,91 @@ def cpu_env(locked_blob, locked_names, nenv, **kw):
     return BatchedLockedEnv(lambda n: OracleBatchedSim(locked_blob, n), m, locked_names, nenv, torch.device("cpu"), **kw)
 
 
-@pytest.fixture(scope="module")
-def ref_modules():
-    for p in (os.path.join(HERE, "stubs"), REF):
-        if p not in sys.path:
-            sys.path.insert(0, p)
-    import robogym_b200.mujoco_py_shim as shim
-
-    shim.install()
-    from oracle_engine import OracleEngine
-
-    shim.set_engine_factory(OracleEngine)
-    yield
-    shim.set_engine_factory(None)
+def golden(name):
+    """what robogym's own LockedEnv / wrappers answered on the mujoco_py shim (tools/make_reference_golden.py)"""
+    return np.load(os.path.join(HERE, "golden", "ref_%s.npz" % name))
 
 
-@needs_reference
-def test_parallel_quats_are_the_reference_set(ref_modules):
-    from robogym.envs.dactyl.common import cube_utils
+def _start_from(b, g):
+    """the batched environment takes the reference environment's state after its reset"""
+    import torch
+
+    b.sim.qpos[0] = torch.tensor(g["qpos"]); b.sim.qvel[0] = torch.tensor(g["qvel"]); b.sim.ctrl[0] = torch.tensor(g["ctrl"])
+    b.sim.pid[0] = torch.tensor(g["pid"]); b.sim.qacc_warmstart[0] = torch.tensor(g["warm"])
+    b.goal_quat[0] = torch.tensor(g["goal_quat"]); b.prev_dist[0] = float(g["prev_dist"])
+    tr = [int(x) for x in g["tracker"]]
+    b.steps_since_last_goal[0], b.consecutive_success[0], b.successes_so_far[0], b.goals_so_far[0], b.success_pending[0] = tr
+
+
+def test_parallel_quats_are_the_reference_set():
     from robogym_b200.locked_env import parallel_quats
 
-    mine, ref = parallel_quats(), np.asarray(cube_utils.PARALLEL_QUATS)
+    mine, ref = parallel_quats(), golden("locked_parallel_quats")["quats"]
     assert mine.shape == ref.shape == (24, 4)
     for q in ref:                       # same set of rotations (q and -q are the same rotation)
         assert min(np.minimum(np.abs(mine - q).max(1), np.abs(mine + q).max(1))) < 1e-9
     assert np.all(mine[:, 0] >= 0) and np.allclose(np.linalg.norm(mine, axis=1), 1.0)
 
 
-@needs_reference
-def test_step_logic_matches_reference_env(ref_modules, locked_blob, locked_names):
+def test_step_logic_matches_reference_env(locked_blob, locked_names):
     """Same state, goal and actions -> same observations, reward terms, done flags and tracker statistics as
     robogym's LockedEnv (no wrappers), through goal successes, a new-goal draw and a per-goal timeout."""
     import torch
 
-    from robogym.envs.dactyl.locked import make_simple_env
-
-    consts = dict(max_timesteps_per_goal=6, successes_needed=2)
-    env = make_simple_env(starting_seed=5, constants=consts)
-    env.reset()
-    sim = env.mujoco_simulation.mj_sim
-    b = cpu_env(locked_blob, locked_names, 1, stop_on_fall=False, auto_reset=False, **consts)
-    d = sim.data
-    b.sim.qpos[0] = torch.tensor(d.qpos.copy()); b.sim.qvel[0] = torch.tensor(d.qvel.copy()); b.sim.ctrl[0] = torch.tensor(d.ctrl.copy())
-    b.sim.pid[0] = torch.tensor(d.userdata[:60].copy()); b.sim.qacc_warmstart[0] = torch.tensor(d.qacc_warmstart.copy())
-    tr = env.multi_goal_tracker
-    b.goal_quat[0] = torch.tensor(env._goal["cube_quat"])
-    b.prev_dist[0] = float(env._previous_goal_distance["cube_quat"])
-    b.steps_since_last_goal[0], b.consecutive_success[0] = tr._steps_since_last_goal, tr._consecutive_steps_with_success
-    b.successes_so_far[0], b.goals_so_far[0], b.success_pending[0] = tr._successes_so_far, tr._goals_so_far, tr._success_and_no_goal_reset
-    rng = np.random.RandomState(1)
+    g = golden("locked_step_logic")
+    b = cpu_env(locked_blob, locked_names, 1, stop_on_fall=False, auto_reset=False, max_timesteps_per_goal=6, successes_needed=2)
+    _start_from(b, g)
     seen = dict(success=0, newgoal=0, timeout=0, trial=0)
-    for k in range(16):
-        if k in (2, 6):   # put the goal on top of the current orientation: the next step succeeds
-            q = d.qpos[env.mujoco_simulation.qpos_idxs["cube_rotation"]].copy()
-            env._goal["cube_quat"] = q
-            env._goal["qpos_goal"][env.mujoco_simulation.qpos_idxs["cube_rotation"]] = q
-            b.goal_quat[0] = torch.tensor(q)
-        a = rng.uniform(-1, 1, 20)
-        obs, rew, done, info = env.step(a)
-        mo, mr, md, mi = b.step(a[None], new_goals=np.asarray(env._goal["cube_quat"])[None])
+    for k in range(len(g["done"])):
+        if not np.isnan(g["goal_override"][k]).any():    # the goal put on top of the current orientation: the next step succeeds
+            b.goal_quat[0] = torch.tensor(g["goal_override"][k])
+        mo, mr, md, mi = b.step(g["action"][k][None], new_goals=g["new_goal"][k][None])
         for key in ("cube_pos", "cube_quat", "hand_angle", "fingertip_pos", "goal_quat", "qpos_goal", "qpos", "qvel"):
-            assert np.abs(mo[key][0].numpy().ravel() - np.asarray(obs[key]).ravel()).max() < 1e-7, (k, key)
-        assert float(mo["is_goal_achieved"][0]) == float(np.asarray(obs["is_goal_achieved"]).ravel()[0]), k
-        assert np.abs(mr[0, :3].numpy() - np.asarray(rew, dtype=float)).max() < 1e-7, (k, rew, mr)
-        assert bool(md[0]) == bool(done), k
-        assert abs(float(mi["goal_dist"][0]) - info["goal_dist"]["cube_quat"]) < 1e-7
+            assert np.abs(mo[key][0].numpy().ravel() - g["obs_" + key][k]).max() < 1e-7, (k, key)
+        assert float(mo["is_goal_achieved"][0]) == float(g["is_goal_achieved"][k]), k
+        assert np.abs(mr[0, :3].numpy() - g["rew"][k]).max() < 1e-7, (k, g["rew"][k], mr)
+        assert bool(md[0]) == bool(g["done"][k]), k
+        assert abs(float(mi["goal_dist"][0]) - g["goal_dist"][k]) < 1e-7
         for key in ("successes_so_far", "goals_so_far", "steps_since_last_goal"):
-            assert int(mi[key][0]) == int(info[key]), (k, key)
+            assert int(mi[key][0]) == int(g[key][k]), (k, key)
         for key in ("trial_success", "sub_goal_is_successful"):
-            assert bool(mi[key][0]) == bool(info[key]), (k, key)
-        seen["success"] += bool(info["sub_goal_is_successful"]); seen["newgoal"] += bool(info.get("goal_reset", False))
-        seen["timeout"] += bool(done and not info["trial_success"]); seen["trial"] += bool(info["trial_success"])
-        if done:
-            break
+            assert bool(mi[key][0]) == bool(g[key][k]), (k, key)
+        seen["success"] += bool(g["sub_goal_is_successful"][k]); seen["newgoal"] += bool(g["goal_reset"][k])
+        seen["timeout"] += bool(g["done"][k] and not g["trial_success"][k]); seen["trial"] += bool(g["trial_success"][k])
     assert seen["success"] == 2 and seen["newgoal"] == 1 and seen["trial"] == 1, seen
 
 
-@needs_reference
-def test_timeout_matches_reference_env(ref_modules, locked_blob, locked_names):
-    import torch
-
-    from robogym.envs.dactyl.locked import make_simple_env
-
-    consts = dict(max_timesteps_per_goal=3, successes_needed=2)
-    env = make_simple_env(starting_seed=2, constants=consts)
-    env.reset()
-    d = env.mujoco_simulation.mj_sim.data
-    b = cpu_env(locked_blob, locked_names, 1, stop_on_fall=False, auto_reset=False, **consts)
-    b.sim.qpos[0] = torch.tensor(d.qpos.copy()); b.sim.qvel[0] = torch.tensor(d.qvel.copy()); b.sim.ctrl[0] = torch.tensor(d.ctrl.copy())
-    b.sim.pid[0] = torch.tensor(d.userdata[:60].copy()); b.sim.qacc_warmstart[0] = torch.tensor(d.qacc_warmstart.copy())
-    b.goal_quat[0] = torch.tensor(env._goal["cube_quat"]); b.prev_dist[0] = float(env._previous_goal_distance["cube_quat"])
-    b.goals_so_far[0] = env.multi_goal_tracker._goals_so_far
-    dones = []
+def test_timeout_matches_reference_env(locked_blob, locked_names):
+    g = golden("locked_timeout")
+    b = cpu_env(locked_blob, locked_names, 1, stop_on_fall=False, auto_reset=False, max_timesteps_per_goal=3, successes_needed=2)
+    _start_from(b, g)
     for k in range(3):
-        a = np.zeros(20)
-        _, rew, done, info = env.step(a)
-        _, mr, md, mi = b.step(a[None])
-        assert bool(md[0]) == bool(done) and np.abs(mr[0, :3].numpy() - np.asarray(rew, dtype=float)).max() < 1e-7
-        dones.append(done)
-    assert dones == [False, False, True]
+        _, mr, md, mi = b.step(np.zeros((1, 20)))
+        assert bool(md[0]) == bool(g["done"][k]) and np.abs(mr[0, :3].numpy() - g["rew"][k]).max() < 1e-7
+    assert list(g["done"]) == [False, False, True]
 
 
-@needs_reference
-def test_reset_randomisation_matches_reference(ref_modules, locked_blob, locked_names):
+def test_reset_randomisation_matches_reference(locked_blob, locked_names):
     """InitialStatePool.randomize with the reference's draws reproduces LockedEnv._randomize_cube_initial_position.
     The random cube pose usually starts in penetration with the fingers, and resolving it amplifies round-off by many
     orders of magnitude per env-step, so the strict comparison uses ONE random-action step; the default ten steps are
     compared through what the reference uses them for (is the cube still on the palm)."""
     import torch
 
-    from robogym.envs.dactyl.locked import make_simple_env
-
-    env = make_simple_env(starting_seed=11)
+    g = golden("locked_reset_randomisation")
     for nrand, tol in ((1, 1e-6), (10, None)):
-        env.parameters.n_random_initial_steps = nrand
         b = cpu_env(locked_blob, locked_names, 1, pool_size=1, n_random_initial_steps=nrand)
         for seed in (3, 4):
-            env._random_state.seed(seed)
-            env.mujoco_simulation.reset()
-            env._randomize_cube_initial_position()
             r = np.random.RandomState(seed)
             wig, quat, act = r.randn(3), r.randn(4), r.uniform(-1.0, 1.0, 20)
             ok = b.pool.randomize(torch.tensor(wig[None]), torch.tensor(quat[None]), torch.tensor(act[None]))
-            d = env.mujoco_simulation.mj_sim.data
+            key = "n%d_seed%d_" % (nrand, seed)
             if tol is not None:
-                assert np.abs(b.pool.sim.qpos[0].numpy() - d.qpos).max() < tol
-                assert np.abs(b.pool.sim.qvel[0].numpy() - d.qvel).max() < 1e-3
+                assert np.abs(b.pool.sim.qpos[0].numpy() - g[key + "qpos"]).max() < tol
+                assert np.abs(b.pool.sim.qvel[0].numpy() - g[key + "qvel"]).max() < 1e-3
             else:
-                assert np.abs(b.pool.sim.qpos[0, 14:].numpy() - d.qpos[14:]).max() < 5e-3     # hand joints
-            assert bool(ok[0]) == bool(env.mujoco_simulation.is_cube_on_palm())
+                assert np.abs(b.pool.sim.qpos[0, 14:].numpy() - g[key + "qpos"][14:]).max() < 5e-3     # hand joints
+            assert bool(ok[0]) == bool(g[key + "on_palm"])
 
 
 def test_cpu_env_success_timeout_and_autoreset(locked_blob, locked_names):
@@ -321,42 +276,26 @@ def test_randomised_env_with_reference_capacities_never_overflows():
     assert worst <= 100
 
 
-@needs_reference
-def test_action_latency_matches_the_reference_wrapper(ref_modules, locked_blob, locked_names):
+def test_action_latency_matches_the_reference_wrapper(locked_blob, locked_names):
     """RandomizedActionLatency (robogym/wrappers/randomizations.py:516-556, first entry of the locked.py:265-277 stack): with
     the same per-coordinate delays, the batched environment hands the simulation the same delayed actions and reports the
     same action_history / action_delay observations as the reference wrapper around the reference env."""
     import torch
 
-    from robogym.envs.dactyl.locked import make_simple_env
-    from robogym.wrappers import randomizations as rz
-
-    inner = make_simple_env(starting_seed=3)
-    performed = []
-    real_step = inner.step
-
-    def spy(action):
-        performed.append(np.array(action, copy=True))
-        return real_step(action)
-
-    inner.step = spy
-    w = rz.RandomizedActionLatency(inner, max_delay=2)
-    obs = w.reset()
+    g = golden("locked_action_latency")
     b = cpu_env(locked_blob, locked_names, 2, stop_on_fall=False, auto_reset=False, action_latency=2)
     b.reset()
     assert b.action_delay.shape == (2, 20) and int(b.action_delay.max()) <= 2 and int(b.action_delay.min()) >= 0
-    b.action_delay[0] = torch.tensor(np.asarray(w._action_delay))
+    b.action_delay[0] = torch.tensor(g["delay"])
     b.action_delay[1] = 0
     sent = []
     orig = b.fac.denormalize_position_control
     b.fac.denormalize_position_control = lambda a, *args, **kw: (sent.append(a.clone()), orig(a, *args, **kw))[1]
-    rng = np.random.RandomState(0)
-    for k in range(6):
-        a = rng.uniform(-1, 1, 20)
-        obs, _, _, _ = w.step(a)
+    for k in range(len(g["action"])):
+        a = g["action"][k]
         mo, _, _, _ = b.step(np.stack([a, a]))
-        assert np.abs(sent[-1][0].numpy() - performed[-1]).max() < 1e-6, k          # env 0: the wrapper's delays
+        assert np.abs(sent[-1][0].numpy() - g["performed"][k]).max() < 1e-6, k      # env 0: the wrapper's delays
         assert np.abs(sent[-1][1].numpy() - a).max() < 1e-6                           # env 1: no delay
-        assert np.abs(mo["action_history"][0].numpy() - np.asarray(obs["action_history"])).max() < 1e-6
-        assert np.array_equal(mo["action_delay"][0].numpy(), np.asarray(obs["action_delay"]))
-    assert len(set(np.asarray(w._action_delay))) > 1, "the fixture drew a single delay: nothing was exercised"
+        assert np.abs(mo["action_history"][0].numpy() - g["action_history"][k]).max() < 1e-6
+        assert np.array_equal(mo["action_delay"][0].numpy(), g["action_delay"][k])
+    assert len(set(g["delay"])) > 1, "the fixture drew a single delay: nothing was exercised"

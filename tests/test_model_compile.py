@@ -75,6 +75,11 @@ def test_mass_matrix_formulations_agree(locked_blob):
 @pytest.mark.skipif(not HAVE_REF, reason="needs /root/reference")
 def test_committed_blob_is_reproducible(locked_blob):
     """tools/compile_models.py on the reference assets reproduces the committed blob bit for bit."""
+    import robogym_b200.mujoco_py_shim as shim
+
+    # the composer falls back to a bare mujoco_py stand-in when none is loaded; the reference modules it imports stay cached
+    # for the rest of the process, so they must bind to the shim the later tests drive them through
+    shim.install()
     import compose_reference_xml as ref
 
     cm = mjcf.compile_mjcf(ref.locked_xml())

@@ -1,45 +1,42 @@
 """robogym_b200/obs_noise.py against the reference's RandomizeObservationWrapper (robogym/wrappers/randomizations.py:314-389): the
-reference wrapper runs on a minimal fake environment with a random state that RECORDS its draws; the batched rule replays exactly
-those draws and must give the same noisy observations, episode biases included."""
+reference wrapper ran on a minimal fake environment with a random state that RECORDED its draws (tests/golden/ref_obs_noise.npz,
+tools/make_reference_golden.py); the batched rule replays exactly those draws and must give the same noisy observations,
+episode biases included."""
 import os
-import sys
 from collections import OrderedDict
 
 import numpy as np
-import pytest
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-REF = os.environ.get("ROBOGYM_REFERENCE", "/root/reference")
-pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "robogym")), reason="needs /root/reference")
+WIDTHS = dict(fingertip_pos=15, hand_angle=24, cube_pos=3, cube_quat=4)
+NENV, NSTEPS = 3, 4
 
 
-class _Recorder:
-    """numpy RandomState look-alike that logs what it hands out"""
-
-    def __init__(self, seed):
-        self.rs, self.log = np.random.RandomState(seed), []
-
-    def randn(self, *shape):
-        v = self.rs.randn(*shape); self.log.append(("randn", v.copy())); return v
-
-    def uniform(self, lo, hi, size=None):
-        v = self.rs.uniform(lo, hi, size=size); self.log.append(("uniform", v.copy())); return v
+def clean_observations():
+    """[step][env] -> the fake environment's clean observation dict"""
+    rng = np.random.RandomState(0)
+    clean = []
+    for s in range(NSTEPS + 1):
+        row = []
+        for e in range(NENV):
+            q = rng.randn(4); q /= np.linalg.norm(q)
+            row.append(OrderedDict(fingertip_pos=rng.randn(15) * 0.05, hand_angle=rng.randn(24) * 0.3, cube_pos=rng.randn(3) * 0.1, cube_quat=q))
+        clean.append(row)
+    return clean
 
 
 class _Replay:
     """the batched rule's `rand`: hands the recorded draws out again, one environment per row"""
 
-    def __init__(self, torch, logs):
-        self.torch, self.logs, self.pos = torch, logs, 0
+    def __init__(self, torch, kinds, sizes, draws):
+        self.torch, self.kinds, self.sizes, self.draws, self.pos, self.off = torch, kinds, sizes, draws, 0, 0
 
     def _next(self, kind, k):
-        vals = []
-        for log in self.logs:
-            what, v = log[self.pos]
-            assert what == kind and v.size == k, (what, kind, v.size, k)
-            vals.append(v.reshape(-1))
+        assert self.kinds[self.pos] == kind and self.sizes[self.pos] == k, (self.kinds[self.pos], kind, self.sizes[self.pos], k)
+        v = self.draws[:, self.off:self.off + k]
         self.pos += 1
-        return self.torch.tensor(np.stack(vals))
+        self.off += k
+        return self.torch.tensor(v)
 
     def randn(self, n, k):
         return self._next("randn", k)
@@ -49,69 +46,25 @@ class _Replay:
 
 
 def test_batched_rule_replays_the_reference_wrapper():
-    for p in (os.path.join(HERE, "stubs"), REF):
-        if p not in sys.path:
-            sys.path.insert(0, p)
-    import robogym_b200.mujoco_py_shim as shim
-
-    shim.install()
-    import gym
     import torch
-    from gym.spaces import Box, Dict
 
-    from robogym.wrappers.randomizations import RandomizeObservationWrapper
     from robogym_b200.obs_noise import LOCKED_LEVELS, BatchedObservationNoise
 
-    widths = dict(fingertip_pos=15, hand_angle=24, cube_pos=3, cube_quat=4)
-    nenv, nsteps = 3, 4
-    rng = np.random.RandomState(0)
-    clean = []                                      # [step][env] -> obs dict
-    for s in range(nsteps + 1):
-        row = []
-        for e in range(nenv):
-            q = rng.randn(4); q /= np.linalg.norm(q)
-            row.append(OrderedDict(fingertip_pos=rng.randn(15) * 0.05, hand_angle=rng.randn(24) * 0.3, cube_pos=rng.randn(3) * 0.1, cube_quat=q))
-        clean.append(row)
-
-    class FakeEnv(gym.Env):
-        def __init__(self, e):
-            self.e, self.k = e, 0
-            self._random_state = _Recorder(100 + e)
-            self.observation_space = Dict({k: Box(-np.inf, np.inf, (w,), np.float64) for k, w in widths.items()})
-            self.action_space = Box(-1, 1, (1,), np.float64)
-
-        @property
-        def unwrapped(self):
-            return self
-
-        def reset(self):
-            self.k = 0
-            return OrderedDict((k, v.copy()) for k, v in clean[0][self.e].items())
-
-        def step(self, a):
-            self.k += 1
-            return OrderedDict((k, v.copy()) for k, v in clean[self.k][self.e].items()), 0.0, False, {}
-
-    envs = [RandomizeObservationWrapper(FakeEnv(e), levels=LOCKED_LEVELS) for e in range(nenv)]
-    ref = [[w.reset() for w in envs]]
-    for s in range(nsteps):
-        ref.append([w.step(np.zeros(1))[0] for w in envs])
-    logs = [w.unwrapped._random_state.log for w in envs]
-
+    g = np.load(os.path.join(HERE, "golden", "ref_obs_noise.npz"))
+    clean = clean_observations()
     rule = BatchedObservationNoise.__new__(BatchedObservationNoise)
-    rule.torch, rule.rand, rule.nenv = torch, _Replay(torch, logs), nenv
-    rule.levels = dict(LOCKED_LEVELS); rule.widths = {k: (1 if k.endswith("_quat") else w) for k, w in widths.items()}
+    rule.torch, rule.rand, rule.nenv = torch, _Replay(torch, [str(k) for k in g["draw_kind"]], g["draw_size"], g["draws"]), NENV
+    rule.levels = dict(LOCKED_LEVELS); rule.widths = {k: (1 if k.endswith("_quat") else w) for k, w in WIDTHS.items()}
     rule.cm = rule.um = 1.0
     rule.additive, rule.multiplicative = {}, {}
     rule.reset()
-    for s in range(nsteps + 1):
-        obs = {k: torch.tensor(np.stack([clean[s][e][k] for e in range(nenv)])) for k in widths}
+    for s in range(NSTEPS + 1):
+        obs = {k: torch.tensor(np.stack([clean[s][e][k] for e in range(NENV)])) for k in WIDTHS}
         got = rule(obs)
-        for k in widths:
-            want = np.stack([ref[s][e]["noisy_" + k] for e in range(nenv)])
-            assert np.abs(got["noisy_" + k].numpy() - want).max() < 1e-12, (s, k)
+        for k in WIDTHS:
+            assert np.abs(got["noisy_" + k].numpy() - g["noisy_" + k][s]).max() < 1e-12, (s, k)
             assert np.array_equal(got[k].numpy(), obs[k].numpy())
-    assert rule.rand.pos == len(logs[0])           # every recorded draw was consumed, in order
+    assert rule.rand.pos == len(g["draw_kind"]) and rule.rand.off == g["draws"].shape[1]   # every recorded draw was consumed, in order
     # the noise is of the documented size: cube position within centimetres, the quaternion a few degrees off
     d = got["noisy_cube_pos"].numpy() - obs["cube_pos"].numpy()
     assert 1e-4 < np.abs(d).max() < 0.05

@@ -2,7 +2,6 @@
 compiler's, the range-perturbation rules against the reference wrappers' own code, the sampled distributions,
 and -- on the GPU -- that the sampled rows reach the engine."""
 import os
-import sys
 
 import numpy as np
 import pytest
@@ -10,8 +9,6 @@ import pytest
 from robogym_b200 import mjcf, modelblob
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-REF = os.environ.get("ROBOGYM_REFERENCE", "/root/reference")
-needs_reference = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "robogym")), reason="needs /root/reference")
 
 
 class NumpyRand:
@@ -104,47 +101,22 @@ def test_sampled_rows_have_the_wrappers_ranges(rnd, locked_names):
     assert hits > 0 and float(x[:, :, 3:].abs().max()) == 0.0 and float(x[:, :R.cube_body].abs().max()) == 0.0
 
 
-@needs_reference
-def test_range_rules_match_reference_wrappers(rnd, locked_names):
+def test_range_rules_match_reference_wrappers(rnd):
     """joint-limit / control-range and tendon-range perturbation: the reference wrappers' own _set_field, run on the
-    shim with the same normal draws, against the batched rules."""
+    shim with given normal draws (tests/golden/ref_range_rules.npz, tools/make_reference_golden.py), against the batched
+    rules fed the same draws."""
     import torch
 
-    for p in (os.path.join(HERE, "stubs"), REF):
-        if p not in sys.path:
-            sys.path.insert(0, p)
-    import robogym_b200.mujoco_py_shim as shim
-
-    shim.install()
-    from oracle_engine import OracleEngine
-
-    shim.set_engine_factory(OracleEngine)
-    try:
-        from robogym.envs.dactyl.locked import make_simple_env
-        from robogym.wrappers import randomizations as rz
-
-        m, R = rnd
-        env = make_simple_env(starting_seed=0)
-        sim = env.unwrapped.sim
-        robot_joints = list(sim.model.joint_names)          # the wrapper's default: every joint
-        jw = rz.RandomizedJointLimitWrapper(env)
-        tw = rz.RandomizedTendonRangeWrapper(env)
-        jw._orig_value = np.array(jw._get_field(sim), copy=True)
-        tw._orig_value = np.array(tw._get_field(sim), copy=True)
-        for seed in (0, 1, 2):
-            r = np.random.RandomState(seed)
-            nj, nt = len(robot_joints), m["ntendon"]
-            zj, zt = r.randn(nj, 2), r.randn(nt, 2)
-            jw._random_noises = lambda n, z=zj: z
-            jw._set_field(sim)
-            env.unwrapped._random_state = type("R", (), {"randn": staticmethod(lambda *s, z=zt: z)})()
-            tw._set_field(sim)
-            got = R.sample(1, noises=dict(joint_limit=torch.tensor(zj[None]), tendon_range=torch.tensor(zt[None])))
-            assert np.abs(got["jnt_range"][0].numpy() - np.asarray(sim.model.jnt_range).ravel()).max() < 1e-12
-            assert np.abs(got["actuator_ctrlrange"][0].numpy() - np.asarray(sim.model.actuator_ctrlrange).ravel()).max() < 1e-12
-            assert np.abs(got["tendon_range"][0].numpy() - np.asarray(sim.model.tendon_range).ravel()).max() < 1e-12
-    finally:
-        shim.set_engine_factory(None)
+    m, R = rnd
+    g = np.load(os.path.join(HERE, "golden", "ref_range_rules.npz"))
+    for seed in (0, 1, 2):
+        key = "seed%d_" % seed
+        zj, zt = g[key + "zj"], g[key + "zt"]
+        assert zt.shape == (m["ntendon"], 2)
+        got = R.sample(1, noises=dict(joint_limit=torch.tensor(zj[None]), tendon_range=torch.tensor(zt[None])))
+        assert np.abs(got["jnt_range"][0].numpy() - g[key + "jnt_range"]).max() < 1e-12
+        assert np.abs(got["actuator_ctrlrange"][0].numpy() - g[key + "actuator_ctrlrange"]).max() < 1e-12
+        assert np.abs(got["tendon_range"][0].numpy() - g[key + "tendon_range"]).max() < 1e-12
 
 
 @pytest.mark.gpu

@@ -1,8 +1,9 @@
 """The batched dual-simulation arm controller (robogym_b200/rearrange_arm.py, SURVEY 8(f) row 4) beside the UNMODIFIED reference
 environment: `robogym.envs.rearrange.blocks.make_env` with ControlMode.TCP_ROLL_YAW + TcpSolverMode.MOCAP_IK (the mode SURVEY
-8(d) row 4 names: 3 tool translations + roll / yaw + gripper) runs on the mujoco_py shim with the oracle as engine; the batched
-controller runs on oracle-backed stand-ins of its two BatchedSims built from the SAME compiled models and started from the SAME
-states.  Both then take the same actions: every env-step must leave the same main-simulation and solver-simulation state
+8(d) row 4 names: 3 tool translations + roll / yaw + gripper) ran on the mujoco_py shim with the oracle as engine and its states
+were recorded (tests/golden/rearrange_arm.json, tests/golden/ref_arm_*.npz); the batched controller runs on oracle-backed
+stand-ins of its two BatchedSims built from the SAME compiled models and started from the SAME states.  Both take the same
+actions: every env-step must leave the same main-simulation and solver-simulation state
 (fp64 on both sides, so the comparison is tight -- any difference is a difference in the control logic).  The GPU test runs the
 controller on two real BatchedSims (CUDA) against the oracle stand-ins, teacher-forced."""
 import os
@@ -12,8 +13,6 @@ import numpy as np
 import pytest
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-REF = os.environ.get("ROBOGYM_REFERENCE", "/root/reference")
-needs_reference = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "robogym")), reason="needs /root/reference")
 for p in (os.path.join(HERE, "stubs"),):
     if p not in sys.path:
         sys.path.insert(0, p)
@@ -22,82 +21,53 @@ MAX_POSITION_CHANGE = float(np.float32(0.1))    # the reference stores the param
 ASSETS = os.path.join(HERE, "..", "robogym_b200", "assets")
 
 
-def _reference_env(reset_controller_error, wrist=False):
-    if REF not in sys.path:
-        sys.path.insert(0, REF)
-    import robogym_b200.mujoco_py_shim as shim
-
-    shim.install()
-    from oracle_engine import OracleEngine
-
-    shim.set_engine_factory(OracleEngine)
-    from robogym.envs.rearrange.blocks import make_env
-    from robogym.robot.robot_interface import ControlMode, TcpSolverMode
-
-    env = make_env(parameters=dict(n_random_initial_steps=0, simulation_params=dict(num_objects=5),
-                                   robot_control_params=dict(control_mode=ControlMode.TCP_WRIST if wrist else ControlMode.TCP_ROLL_YAW, tcp_solver_mode=TcpSolverMode.MOCAP_IK,
-                                                             arm_reset_controller_error=reset_controller_error,
-                                                             max_position_change=MAX_POSITION_CHANGE)), starting_seed=0)
-    env.reset()
-    return env.unwrapped, shim          # the environment itself, below the action wrappers (discretisation, smoothing): continuous actions
+def _recorded(name):
+    """what the reference environment's two simulations did on the mujoco_py shim (tools/make_reference_golden.py)"""
+    return np.load(os.path.join(HERE, "golden", "ref_%s.npz" % name))
 
 
-def _copy_state(sim_stub, mj_sim):
-    import torch
-
-    d = mj_sim.data
-    w = sim_stub.pid.shape[1]
-    sim_stub.qpos[:] = torch.tensor(d.qpos); sim_stub.qvel[:] = torch.tensor(d.qvel); sim_stub.ctrl[:] = torch.tensor(d.ctrl)
-    sim_stub.pid[:] = torch.tensor(d.userdata[:w]); sim_stub.qacc_warmstart[:] = torch.tensor(d.qacc_warmstart)
-    if sim_stub.mocap_pos is not None:
-        sim_stub.mocap_pos[:] = torch.tensor(d.mocap_pos); sim_stub.mocap_quat[:] = torch.tensor(d.mocap_quat)
-    sim_stub.body_xpos[:] = torch.tensor(d.body_xpos); sim_stub.body_xquat[:] = torch.tensor(d.body_xquat)
+def _state_of(g, prefix, sim):
+    """one recorded simulation state in the layout _load_state takes"""
+    st = {k: g[prefix + k] for k in ("qpos", "qvel", "ctrl", "warm", "body_xpos", "body_xquat")}
+    st["pid"] = g[prefix + "pid"][:sim.pid.shape[1]]
+    if sim.mocap_pos is not None:
+        st.update(mocap_pos=g[prefix + "mocap_pos"], mocap_quat=g[prefix + "mocap_quat"])
+    return st
 
 
-@needs_reference
 @pytest.mark.parametrize("reset_controller_error", [True, False])
 def test_batched_controller_steps_like_the_reference_environment(reset_controller_error):
+    """Two environments in one batch from the reference environment's recorded reset state: every env-step reproduces the
+    recorded main / solver states and controls (fp64 on both sides), and the batch rows agree bit for bit."""
     import torch
 
     from oracle_generic_sim import OracleGenericSim
     from robogym_b200.rearrange_arm import BatchedTcpArmController
 
-    env, shim = _reference_env(reset_controller_error)
-    try:
-        main_mj = env.mujoco_simulation.mj_sim
-        arm = env.robot.robots[0]
-        solver_mj = arm.controller_arm.mj_sim
-        assert type(arm).__name__ == "JointControlledTcpArm" and type(arm.controller_arm).__name__ == "FreeRollYawTcpArm"
-        nenv = 2
-        main = OracleGenericSim(main_mj.model._cm.blob(), nenv, main_mj.nsubsteps)
-        solver = OracleGenericSim(solver_mj.model._cm.blob(), nenv, solver_mj.nsubsteps)
-        assert main.model.host["nu"] == 7 and list(main.model.host["actuator_user0"]) == [1, 1, 1, 1, 1, 1, 0]    # cascaded-PI arm, PID gripper
-        assert solver.model.host["nmocap"] == 1 and solver.model.host["neq"] == 2        # mocap weld + gripper coupling
-        _copy_state(main, main_mj)
-        _copy_state(solver, solver_mj)
-        ctl = BatchedTcpArmController(main, solver, MAX_POSITION_CHANGE, reset_controller_error=reset_controller_error)
-        assert ctl.action_dim == env.action_space.shape[0] == 6
-        rng = np.random.RandomState(0)
-        worst = 0.0
-        for k in range(12):
-            a = rng.uniform(-1, 1, 6).astype(np.float32)   # the environment's action space is float32
-            if k == 5:
-                a[4] = 1.0                  # push the wrist towards its range: exercises constrain_quat_ctrl
-            env.step(a)
-            ctl.step(torch.tensor(np.stack([a, a])))
-            em = np.abs(main.qpos[0].numpy() - main_mj.data.qpos).max()
-            es = np.abs(solver.qpos[0].numpy() - solver_mj.data.qpos).max()
-            ec = np.abs(main.ctrl[0].numpy() - main_mj.data.ctrl).max()
-            emo = np.abs(solver.mocap_pos[0].numpy() - solver_mj.data.mocap_pos).max()
-            worst = max(worst, em, es, ec, emo)
-            assert em < 1e-9 and es < 1e-9 and ec < 1e-9 and emo < 1e-9, (k, em, es, ec, emo)
-            assert torch.equal(main.qpos[0], main.qpos[1])
-        assert worst < 1e-9 and int(main.warn.max()) == 0
-    finally:
-        shim.set_engine_factory(None)
+    fx, blobs = _fixture()
+    rec = fx["reset_error_%s" % str(reset_controller_error).lower()]
+    assert rec["reset_controller_error"] == reset_controller_error and len(rec["actions"][0]) == 6
+    nenv = 2
+    main = OracleGenericSim(blobs[0], nenv, rec["nsub_main"])
+    solver = OracleGenericSim(blobs[1], nenv, rec["nsub_solver"])
+    assert main.model.host["nu"] == 7 and list(main.model.host["actuator_user0"]) == [1, 1, 1, 1, 1, 1, 0]    # cascaded-PI arm, PID gripper
+    assert solver.model.host["nmocap"] == 1 and solver.model.host["neq"] == 2        # mocap weld + gripper coupling
+    _load_state(main, rec["main0"]); _load_state(solver, rec["solver0"])
+    ctl = BatchedTcpArmController(main, solver, MAX_POSITION_CHANGE, reset_controller_error=reset_controller_error)
+    assert ctl.action_dim == 6
+    worst = 0.0
+    for k, a in enumerate(rec["actions"]):
+        ctl.step(torch.tensor([a, a], dtype=torch.float32))
+        em = np.abs(main.qpos[0].numpy() - rec["main_qpos"][k]).max()
+        es = np.abs(solver.qpos[0].numpy() - rec["solver_qpos"][k]).max()
+        ec = np.abs(main.ctrl[0].numpy() - rec["main_ctrl"][k]).max()
+        emo = np.abs(solver.mocap_pos[0].numpy() - np.asarray(rec["solver_mocap_pos"][k])).max()
+        worst = max(worst, em, es, ec, emo)
+        assert em < 1e-9 and es < 1e-9 and ec < 1e-9 and emo < 1e-9, (k, em, es, ec, emo)
+        assert torch.equal(main.qpos[0], main.qpos[1])
+    assert worst < 1e-9 and int(main.warn.max()) == 0
 
 
-@needs_reference
 def test_wrist_mode_with_its_alignment_axis_steps_like_the_reference_environment():
     """ControlMode.TCP_WRIST: one tool rotation (about the vertical), the commanded orientation re-aligned with the vertical
     axis every step (MocapSolver.align_axis)."""
@@ -106,57 +76,43 @@ def test_wrist_mode_with_its_alignment_axis_steps_like_the_reference_environment
     from oracle_generic_sim import OracleGenericSim
     from robogym_b200.rearrange_arm import BatchedTcpArmController
 
-    env, shim = _reference_env(True, wrist=True)
-    try:
-        main_mj = env.mujoco_simulation.mj_sim
-        arm = env.robot.robots[0]
-        solver_mj = arm.controller_arm.mj_sim
-        assert type(arm.controller_arm).__name__ == "FreeWristTcpArm" and env.action_space.shape[0] == 5
-        main = OracleGenericSim(main_mj.model._cm.blob(), 1, main_mj.nsubsteps)
-        solver = OracleGenericSim(solver_mj.model._cm.blob(), 1, solver_mj.nsubsteps)
-        _copy_state(main, main_mj)
-        _copy_state(solver, solver_mj)
-        ctl = BatchedTcpArmController(main, solver, MAX_POSITION_CHANGE, dof_dims=("pitch",), align_axis="pitch")
-        assert ctl.action_dim == 5
-        rng = np.random.RandomState(1)
-        for k in range(8):
-            a = rng.uniform(-1, 1, 5).astype(np.float32)
-            env.step(a)
-            ctl.step(torch.tensor(a[None]))
-            em = np.abs(main.qpos[0].numpy() - main_mj.data.qpos).max()
-            es = np.abs(solver.qpos[0].numpy() - solver_mj.data.qpos).max()
-            eq = np.abs(solver.mocap_quat[0].numpy() - solver_mj.data.mocap_quat).max()
-            assert em < 1e-9 and es < 1e-9 and eq < 1e-9, (k, em, es, eq)
-    finally:
-        shim.set_engine_factory(None)
+    g = _recorded("arm_wrist")
+    _, blobs = _fixture()
+    main = OracleGenericSim(blobs[0], 1, int(g["nsub_main"]))
+    solver = OracleGenericSim(blobs[1], 1, int(g["nsub_solver"]))
+    _load_state(main, _state_of(g, "main0_", main))
+    _load_state(solver, _state_of(g, "solver0_", solver))
+    ctl = BatchedTcpArmController(main, solver, MAX_POSITION_CHANGE, dof_dims=("pitch",), align_axis="pitch")
+    assert ctl.action_dim == g["action"].shape[1] == 5
+    for k, a in enumerate(g["action"]):
+        ctl.step(torch.tensor(a[None]))
+        em = np.abs(main.qpos[0].numpy() - g["main_qpos"][k]).max()
+        es = np.abs(solver.qpos[0].numpy() - g["solver_qpos"][k]).max()
+        eq = np.abs(solver.mocap_quat[0].numpy() - g["solver_mocap_quat"][k]).max()
+        assert em < 1e-9 and es < 1e-9 and eq < 1e-9, (k, em, es, eq)
 
 
-@needs_reference
 def test_controller_reset_reseats_the_mocap_weld_like_the_reference():
     import torch
 
     from oracle_generic_sim import OracleGenericSim
     from robogym_b200.rearrange_arm import BatchedTcpArmController
 
-    env, shim = _reference_env(True)
-    try:
-        main_mj = env.mujoco_simulation.mj_sim
-        solver_mj = env.robot.robots[0].controller_arm.mj_sim
-        main = OracleGenericSim(main_mj.model._cm.blob(), 1, main_mj.nsubsteps)
-        solver = OracleGenericSim(solver_mj.model._cm.blob(), 1, solver_mj.nsubsteps)
-        _copy_state(main, main_mj)
-        # the solver stand-in starts from its MODEL state (qpos0, compiled weld pose); reset() must bring it to the reference's
-        solver.model.set_field("eq_data", np.tile([0.1, 0.0, 0.0, 1.0, 0.0, 0.0, 0.0], int(solver.model.host["neq"])))
-        ctl = BatchedTcpArmController(main, solver, MAX_POSITION_CHANGE)
-        ctl.reset()
-        weld = [i for i in range(int(solver.model.host["neq"])) if int(solver.model.host["eq_type"][i]) == 1]
-        assert np.allclose(np.asarray(solver.model.host["eq_data"]).reshape(int(solver.model.host["neq"]), -1)[weld, :7], [0, 0, 0, 1, 0, 0, 0])
-        assert np.abs(solver.qpos[0, ctl.arm_qadr_solver].numpy() - main_mj.data.qpos[ctl.arm_qadr_main]).max() == 0
-        tcp = solver.model.name2id("body", "robot0:gripper_tcp")
-        assert torch.equal(solver.mocap_pos[0, 0], solver.body_xpos[0, tcp]) and torch.equal(solver.mocap_quat[0, 0], solver.body_xquat[0, tcp])
-        assert np.abs(solver.mocap_pos[0, 0].numpy() - solver_mj.data.mocap_pos[0]).max() < 2e-3   # the reference's helper arm has drifted a little by then
-    finally:
-        shim.set_engine_factory(None)
+    g = _recorded("arm_reset")
+    _, blobs = _fixture()
+    main = OracleGenericSim(blobs[0], 1, int(g["nsub_main"]))
+    solver = OracleGenericSim(blobs[1], 1, int(g["nsub_solver"]))
+    _load_state(main, _state_of(g, "main0_", main))
+    # the solver stand-in starts from its MODEL state (qpos0, compiled weld pose); reset() must bring it to the reference's
+    solver.model.set_field("eq_data", np.tile([0.1, 0.0, 0.0, 1.0, 0.0, 0.0, 0.0], int(solver.model.host["neq"])))
+    ctl = BatchedTcpArmController(main, solver, MAX_POSITION_CHANGE)
+    ctl.reset()
+    weld = [i for i in range(int(solver.model.host["neq"])) if int(solver.model.host["eq_type"][i]) == 1]
+    assert np.allclose(np.asarray(solver.model.host["eq_data"]).reshape(int(solver.model.host["neq"]), -1)[weld, :7], [0, 0, 0, 1, 0, 0, 0])
+    assert np.abs(solver.qpos[0, ctl.arm_qadr_solver].numpy() - g["main0_qpos"][ctl.arm_qadr_main]).max() == 0
+    tcp = solver.model.name2id("body", "robot0:gripper_tcp")
+    assert torch.equal(solver.mocap_pos[0, 0], solver.body_xpos[0, tcp]) and torch.equal(solver.mocap_quat[0, 0], solver.body_xquat[0, tcp])
+    assert np.abs(solver.mocap_pos[0, 0].numpy() - g["solver_mocap_pos"][0]).max() < 2e-3   # the reference's helper arm has drifted a little by then
 
 
 # ---- the same comparison from the committed fixture (tools/make_rearrange_arm_fixture.py): no reference needed, and the GPU tier
@@ -377,52 +333,24 @@ def test_recorded_impulse_response_on_cuda():
     _assert_impulse(_impulse_response(make, device="cuda:0", sync=torch.cuda.synchronize))
 
 
-@needs_reference
 def test_batched_controller_steps_like_the_reference_ycb_environment():
     """BASELINE configs[4]: the reference's ycb environment (8 mesh objects of its own draw, the first starting_seed whose
-    placement succeeds) beside the batched controller on stand-ins built from the environment's compiled models."""
+    placement succeeds; its main simulation is the committed rearrange_ycb8_tcp asset) beside the batched controller."""
     import torch
 
     from oracle_generic_sim import OracleGenericSim
     from robogym_b200.rearrange_arm import BatchedTcpArmController
 
-    if REF not in sys.path:
-        sys.path.insert(0, REF)
-    import robogym_b200.mujoco_py_shim as shim
-
-    shim.install()
-    from oracle_engine import OracleEngine
-
-    shim.set_engine_factory(OracleEngine)
-    try:
-        from robogym.envs.rearrange.ycb import make_env
-        from robogym.robot.robot_interface import ControlMode, TcpSolverMode
-
-        env = make_env(parameters=dict(n_random_initial_steps=0, simulation_params=dict(num_objects=8, max_num_objects=8),
-                                       robot_control_params=dict(control_mode=ControlMode.TCP_ROLL_YAW, tcp_solver_mode=TcpSolverMode.MOCAP_IK,
-                                                                 max_position_change=MAX_POSITION_CHANGE)),
-                       constants=dict(stabilize_objects=False), starting_seed=1)
-        env.reset()
-        env = env.unwrapped
-        main_mj = env.mujoco_simulation.mj_sim
-        solver_mj = env.robot.robots[0].controller_arm.mj_sim
-        blob = main_mj.model._cm.blob()
-        # the committed bench asset is this environment's main simulation (tools/make_rearrange_ycb_tcp_asset.py)
-        asset = open(os.path.join(ASSETS, "rearrange_ycb8_tcp.rgm"), "rb").read()
-        assert len(asset) == len(blob)
-        main = OracleGenericSim(blob, 1, main_mj.nsubsteps)
-        solver = OracleGenericSim(solver_mj.model._cm.blob(), 1, solver_mj.nsubsteps)
-        assert (main.model.host["nq"], main.model.host["nv"], main.model.host["nu"]) == (64, 56, 7)
-        _copy_state(main, main_mj)
-        _copy_state(solver, solver_mj)
-        ctl = BatchedTcpArmController(main, solver, MAX_POSITION_CHANGE)
-        rng = np.random.RandomState(2)
-        for k in range(5):
-            a = rng.uniform(-1, 1, 6).astype(np.float32)
-            env.step(a)
-            ctl.step(torch.tensor(a[None]))
-            em = np.abs(main.qpos[0].numpy() - main_mj.data.qpos).max()
-            es = np.abs(solver.qpos[0].numpy() - solver_mj.data.qpos).max()
-            assert em < 1e-9 and es < 1e-9, (k, em, es)
-    finally:
-        shim.set_engine_factory(None)
+    g = _recorded("arm_ycb")
+    blob = open(os.path.join(ASSETS, "rearrange_ycb8_tcp.rgm"), "rb").read()
+    main = OracleGenericSim(blob, 1, int(g["nsub_main"]))
+    solver = OracleGenericSim(_fixture()[1][1], 1, int(g["nsub_solver"]))
+    assert (main.model.host["nq"], main.model.host["nv"], main.model.host["nu"]) == (64, 56, 7)
+    _load_state(main, _state_of(g, "main0_", main))
+    _load_state(solver, _state_of(g, "solver0_", solver))
+    ctl = BatchedTcpArmController(main, solver, MAX_POSITION_CHANGE)
+    for k, a in enumerate(g["action"]):
+        ctl.step(torch.tensor(a[None]))
+        em = np.abs(main.qpos[0].numpy() - g["main_qpos"][k]).max()
+        es = np.abs(solver.qpos[0].numpy() - g["solver_qpos"][k]).max()
+        assert em < 1e-9 and es < 1e-9, (k, em, es)
